@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RGB-D pair frames/sec of the se(3)-TrackNet per-frame hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64] [--precision tf32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64] [--precision tf32] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of synthetic input: `batch` (default 64)
@@ -23,6 +23,8 @@ Prints ONE JSON line (rank 0).  Keys beyond the base contract:
                 poses, rendered views and D2H of the poses inside every timed step
 --impl reference: the reference's own CPU implementation of the path (oracle restatement: the
 reference code itself cannot travel to the GPU box) on all host threads, bounded sample per step.
+--dump-outputs DIR: after the timed steps, the poses the last timed step returned go to DIR/poses.npy (float64, one 4x4 per
+track; with N > 1 also DIR/poses_all_ranks.npy, the gathered set).  Inputs are seeded: the same arguments give the same inputs.
 """
 import argparse, importlib, json, os, subprocess, sys, threading, time
 import numpy as np
@@ -49,10 +51,24 @@ def parse():
     ap.add_argument('--no-render', action='store_true', help='skip the step-with-rendered-input-A measurement')
     ap.add_argument('--no-g21', action='store_true', help='skip the 21-weight-set leg')
     ap.add_argument('--cpu-seconds', type=float, default=12.0)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the poses the last timed step returned (rank 0) as DIR/<name>.npy')
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.impl == 'reference' else 500
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     return args
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be
+    compared file for file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def workload_string(nb):
@@ -188,8 +204,10 @@ def run_reference(args, synth, rank, world):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        last = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'poses': np.stack(last)})
     val = args.steps * per_step / dt
     sample = 'each step = all %d pairs of the workload (per-pair numpy/cv2 crop + normalise, ONE batched torch CPU forward, per-pair pose update); %d steps' % (per_step, args.steps)
     line = {'impl': 'reference', 'metric': 'rgbd_pair_frames_per_sec', 'value': val, 'unit': 'pairs/s', 'n_gpus': args.gpus,
@@ -274,13 +292,17 @@ def main():
     for k in range(args.steps):
         flush.zero_()                                   # evict the previous step's lines from L2 (untimed)
         ev[k][0].record()
-        step(k)
+        last = step(k)
         ev[k][1].record()
         launches += eng.last_launch_count()
     # the last step's pose all-gather runs on the side stream: its completion belongs to the timed region too
     tail = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
     tail[0].record(); tracker.wait_gather(); tail[1].record()
     sync_all()
+    if args.dump_outputs and rank == 0:          # before later steps reuse the tracker's output buffers
+        mine, gathered = last
+        dump_outputs(args.dump_outputs, {'poses': mine.cpu().numpy()} if gathered is None else
+                     {'poses': mine.cpu().numpy(), 'poses_all_ranks': gathered.cpu().numpy()})
     ms_steps = np.array([a.elapsed_time(b) for a, b in ev])
     total_ms = torch.tensor([float(ms_steps.sum()) + tail[0].elapsed_time(tail[1])], device=dev)
     if world > 1:
@@ -541,4 +563,5 @@ def main():
 
 
 if __name__ == '__main__':
+    sys.dont_write_bytecode = True          # the tree may be read-only: a benchmark run leaves it exactly as it found it
     main()
